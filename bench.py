@@ -88,7 +88,12 @@ def parse_args():
     p.add_argument("--no-gpu-numa", action="store_true")
     p.add_argument("--kernel-block-kib", type=int, default=0,
                    help="block size of the kernel-level window (0 = the config's block size)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step computed to "
+                        "DIR/<name>.npy (see dump_outputs)")
     args = p.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
     if args.threads <= 0:
         args.threads = max(1, min(16, int(cpu_quota() // max(1, args.gpus))))
     return args
@@ -318,6 +323,10 @@ class Workload:
     def cleanup_paths(self, rank):
         return []
 
+    def written_regions(self, step, rank):
+        """[(path, offset, length)] of the file data that step writes on behalf of `rank`"""
+        return []
+
     def common_cfg(self):
         return dict(block_size=self.block, use_direct_io=self.args.direct)
 
@@ -358,6 +367,11 @@ class SeqFileWorkload(Workload):
 
     def cleanup_paths(self, rank):
         return [self.paths[rank]]
+
+    def written_regions(self, step, rank):
+        if not self.do_write_in_step:
+            return []
+        return [(self.paths[rank], step * self.slice_bytes, self.slice_bytes)]
 
 
 class C2(SeqFileWorkload):
@@ -483,6 +497,12 @@ class C5(Workload):
     def cleanup_paths(self, rank):
         return [self.step_dir(s) for s in range(self.num_slices)] if rank == 0 else []
 
+    def written_regions(self, step, rank):
+        """every file of the step's tree (the ranks share it), in path order"""
+        files = sorted(os.path.join(root, name) for root, _, names in os.walk(self.step_dir(step))
+                       for name in names)
+        return [(path, 0, os.path.getsize(path)) for path in files]
+
 
 WORKLOADS = {"c2": C2, "c3": C3, "c4": C4, "c5": C5}
 TIMED_PHASES = ("CREATEFILES", "READFILES")  # (mkdirs of c5 are preparation of the step)
@@ -524,6 +544,55 @@ def phase_rates(totals):
         if ph["entries"]:
             out[short + "_files_s"] = int(ph["entries"] / secs)
     return out
+
+
+DUMP_SEED = 20240531
+DUMP_CHUNKS = 256
+DUMP_CHUNK_BYTES = 4096
+
+
+def dump_outputs(out_dir, workload, step, rank, step_results):
+    """Write what timed step `step` computed, so that two builds can be compared output for
+    output on the same arguments:
+      <phase>_counters.npy      float64 [entries, bytes, iops, verified bytes, verify mismatch
+                                bytes, filled bytes] of each timed phase (the job-wide results the
+                                caller receives; times and latencies are left out, they differ
+                                from run to run)
+      written_sample.npy        float32 [DUMP_CHUNKS, chunk] bytes of the file data the step wrote,
+                                at offsets drawn with a fixed seed (configs whose steps write)
+      written_sample_where.npy  float64 [DUMP_CHUNKS, 2] (region index, offset in region) of each
+                                row, regions in the order of workload.written_regions()
+    At most 4 MiB in all."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, res in step_results.items():
+        if name not in TIMED_PHASES:
+            continue
+        ops = res["ops_total"]
+        counters = [ops["entries"], ops["bytes"], ops["iops"], res["verified_bytes"],
+                    res["verify_mismatch_bytes"], res["filled_bytes"]]
+        np.save(os.path.join(out_dir, name.lower() + "_counters.npy"),
+                np.array(counters, dtype=np.float64))
+    regions = workload.written_regions(step, rank)
+    if not regions:
+        return
+    lengths = np.array([length for _, _, length in regions], dtype=np.int64)
+    chunk = int(min(DUMP_CHUNK_BYTES, lengths.min()))
+    rng = np.random.default_rng(DUMP_SEED)
+    picks = rng.choice(len(regions), size=DUMP_CHUNKS, p=lengths / lengths.sum())
+    offsets = rng.integers(0, lengths[picks] - chunk, endpoint=True)
+    sample = np.empty((DUMP_CHUNKS, chunk), dtype=np.float32)
+    for row, (idx, off) in enumerate(zip(picks, offsets)):
+        path, start, _ = regions[idx]
+        with open(path, "rb") as f:
+            f.seek(start + int(off))
+            data = f.read(chunk)
+        if len(data) != chunk:
+            raise RuntimeError("short read of %s at %d" % (path, start + int(off)))
+        sample[row] = np.frombuffer(data, dtype=np.uint8)
+    np.save(os.path.join(out_dir, "written_sample.npy"), sample)
+    np.save(os.path.join(out_dir, "written_sample_where.npy"),
+            np.stack([picks, offsets], axis=1).astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -876,7 +945,7 @@ def gpu_arm(args, torch, device, workload, rank):
             if src["num"]:
                 histo["min_usec"] = min(histo["min_usec"], src["min_usec"])
                 histo["max_usec"] = max(histo["max_usec"], src["max_usec"])
-    return totals, extra, prep_info
+    return totals, extra, prep_info, res
 
 
 def pool_steps(workload, world, warmup, steps):
@@ -1153,7 +1222,10 @@ def main():
 
     sampler = ClockSampler(local_rank).start() if rank == 0 else None
     try:
-        totals, extra, prep_info = gpu_arm(args, torch, device, workload, rank)
+        totals, extra, prep_info, last_step = gpu_arm(args, torch, device, workload, rank)
+        if args.dump_outputs and rank == 0:  # (before the cleanup removes the written files)
+            dump_outputs(args.dump_outputs, workload, args.warmup + args.steps - 1, rank,
+                         last_step)
     finally:
         barrier(torch, device)
         remove_paths(workload.cleanup_paths(rank))

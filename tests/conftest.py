@@ -19,13 +19,12 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The reference's own headers behind a C ABI (oracle/_ref/libelb_ref.so), or skip."""
-    from tests import oracle_lib
-    lib = oracle_lib.load_ref()
-    if lib is None:
-        pytest.skip("oracle/_ref/libelb_ref.so not built (reference tree absent)")
-    return lib
+def recorded():
+    """The reference's answers to the seeded cases of tests/golden/make_golden.py
+    (tests/golden/ref_recorded.json)."""
+    import json
+    with open(os.path.join(REPO_ROOT, "tests", "golden", "ref_recorded.json")) as f:
+        return json.load(f)
 
 
 @pytest.fixture(scope="session")

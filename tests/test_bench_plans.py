@@ -92,6 +92,43 @@ def test_c5_counts_files_and_reads_them_back(workdir):
     assert totals["phase"]["READFILES"]["bytes"] == files_per_step * args.steps * workload.block
 
 
+@pytest.mark.parametrize("name", ["c2", "c5"])
+def test_dump_outputs_samples_what_the_last_step_wrote(workdir, tmp_path, name):
+    import numpy as np
+    args = make_args(workdir, config=name, file_gib=(24 if name == "c2" else 64) / 1024)
+    workload = bench.WORKLOADS[name](args, 1)
+    bench.cpu_arm(workload, args.steps, args.warmup)
+    last = args.warmup + args.steps - 1
+    counters = {"ops_total": {"entries": 3, "bytes": 4 << 20, "iops": 4}, "verified_bytes": 7,
+                "verify_mismatch_bytes": 0, "filled_bytes": 4 << 20}
+    step_results = {"CREATEDIRS": counters, "CREATEFILES": counters, "READFILES": counters}
+    dumps = [tmp_path / "a", tmp_path / "b"]
+    for out in dumps:
+        bench.dump_outputs(str(out), workload, last, 0, step_results)
+    names = sorted(os.listdir(dumps[0]))
+    assert names == ["createfiles_counters.npy", "readfiles_counters.npy", "written_sample.npy",
+                     "written_sample_where.npy"]
+    total = 0
+    for fname in names:
+        a, b = np.load(dumps[0] / fname), np.load(dumps[1] / fname)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)  # seeded: repeatable
+        total += a.nbytes
+    assert total <= 64 << 20
+    assert np.load(dumps[0] / "readfiles_counters.npy").tolist() == [3, 4 << 20, 4, 7, 0, 4 << 20]
+    sample = np.load(dumps[0] / "written_sample.npy")
+    where = np.load(dumps[0] / "written_sample_where.npy").astype(np.int64)
+    regions = workload.written_regions(last, 0)
+    assert sample.shape == (bench.DUMP_CHUNKS, min(bench.DUMP_CHUNK_BYTES,
+                                                   min(r[2] for r in regions)))
+    if name == "c2":
+        assert regions == [(workload.paths[0], last * workload.slice_bytes, workload.slice_bytes)]
+    for row, (idx, off) in zip(sample, where):
+        path, start, length = regions[idx]
+        assert 0 <= off <= length - sample.shape[1]
+        want = oracle_lib.fill_pattern(sample.shape[1], start + off, args.salt)
+        assert row.astype(np.uint8).tobytes() == want
+
+
 @pytest.mark.parametrize("name", ["c2", "c3", "c4", "c5"])
 @pytest.mark.parametrize("world", [1, 8])
 def test_b200_arm_json_line_from_fake_measurements(workdir, name, world):

@@ -139,20 +139,22 @@ def test_partition_matches_reference_pathstore_golden(native, tmp_path):
                 assert buf.value.decode() == want[name], (case["numDataSetThreads"], rank, name)
 
 
-def test_partition_live_against_reference_pathstore(native, ref, tmp_path):
-    rng = random.Random(2024)
-    buf_a = ctypes.create_string_buffer(1 << 20)
-    buf_b = ctypes.create_string_buffer(1 << 20)
-    for round_idx in range(6):
-        block = rng.choice([4 * KiB, 64 * KiB, 1000])
+def test_partition_live_against_reference_pathstore(native, recorded, tmp_path):
+    """random trees against the reference's own PathStore.cpp (digests of its dir and file lists
+    per worker, recorded by tests/golden/make_golden.py)"""
+    from tests.golden import make_golden
+    cases = make_golden.custom_tree_cases()
+    assert len(cases) == len(recorded["custom_trees"])
+    buf = ctypes.create_string_buffer(1 << 20)
+    for round_idx, ((block, tree_text, splits), want) in enumerate(
+            zip(cases, recorded["custom_trees"])):
         tree_path = tmp_path / ("tree%d.txt" % round_idx)
-        tree_path.write_text(make_tree_text(rng, 60, 10, block))
-        for nthreads in (1, 2, 5, 16):
-            for share, round_up in ((0, 0), (4 * block, 0), (0, 512)):
-                for rank in range(nthreads):
-                    for kind in (0, 1):
-                        args = (str(tree_path).encode(), block, share, round_up, rank, nthreads,
-                                kind)
-                        assert native.elb_custom_tree_worker_list(*args, buf_a, len(buf_a)) >= 0
-                        assert ref.ref_custom_tree_worker_list(*args, buf_b, len(buf_b)) >= 0
-                        assert buf_a.value == buf_b.value, (block, nthreads, share, round_up, rank)
+        tree_path.write_text(tree_text)
+        for (nthreads, share, round_up), digests in zip(splits, want):
+            got = []
+            for rank in range(nthreads):
+                for kind in (0, 1):
+                    args = (str(tree_path).encode(), block, share, round_up, rank, nthreads, kind)
+                    assert native.elb_custom_tree_worker_list(*args, buf, len(buf)) >= 0
+                    got.append(make_golden.tree_list_digest(buf.value.decode()))
+            assert got == digests, (block, nthreads, share, round_up)

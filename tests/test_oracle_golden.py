@@ -1,6 +1,6 @@
 """Pin the CPU oracle: against the committed golden vectors generated from the reference's own
-headers (tests/golden/ref_vectors.json) and, when oracle/_ref/libelb_ref.so is present, live
-against those headers on additional random cases. No GPU needed."""
+headers (tests/golden/ref_vectors.json) and against those headers' answers to additional seeded
+random cases (tests/golden/ref_recorded.json). No GPU needed."""
 import ctypes
 import hashlib
 import json
@@ -10,6 +10,7 @@ import random
 import pytest
 
 from tests import oracle_lib
+from tests.golden import make_golden
 from tests.golden.make_golden import pattern_closed_form
 
 GOLDEN_PATH = os.path.join(os.path.dirname(__file__), "golden", "ref_vectors.json")
@@ -152,21 +153,20 @@ def test_offsetgen_randalgo_golden(oracle, golden):
         assert [list(x) for x in seq] == vec["sequence"], (vec["algo"], vec["kind"])
 
 
-def test_randalgo_live_vs_reference_headers(oracle, ref):
-    rng = random.Random(99)
-    for algo_id in (0, 1, 2, 3):
-        for _ in range(5):
-            state = [rng.getrandbits(64) for _ in range(4)]
-            a = oracle.orc_randalgo_create(algo_id, oracle_lib.u64x4(state))
-            b = ref.ref_randalgo_create(algo_id, oracle_lib.u64x4(state))
-            assert [oracle.orc_randalgo_next(a) for _ in range(1000)] == \
-                [ref.ref_randalgo_next(b) for _ in range(1000)], algo_id
-            oracle.orc_randalgo_destroy(a)
-            ref.ref_randalgo_destroy(b)
-            for kind in (2, 3):
-                args = (kind, 50 * 4096 + 5, 1 << 20, 8192, 4096, 1, state, 0)
-                assert oracle_lib.offsetgen_sequence(oracle, "orc", *args, rand_algo=algo_id) == \
-                    oracle_lib.offsetgen_sequence(ref, "ref", *args, rand_algo=algo_id)
+def test_randalgo_live_vs_reference_headers(oracle, recorded):
+    """random injected states against the answers of the reference's headers
+    (recorded by tests/golden/make_golden.py)"""
+    cases = make_golden.randalgo_cases()
+    assert len(cases) == len(recorded["randalgo"])
+    for (algo_id, state), want in zip(cases, recorded["randalgo"]):
+        algo = oracle.orc_randalgo_create(algo_id, oracle_lib.u64x4(state))
+        nexts = [oracle.orc_randalgo_next(algo) for _ in range(1000)]
+        oracle.orc_randalgo_destroy(algo)
+        assert nexts[:8] == want["next8"], algo_id
+        assert make_golden.u64_digest(nexts) == want["next1000_sha256"], algo_id
+        for args, seq in zip(make_golden.RANDALGO_OFFSETGEN_ARGS, want["offsetgen_sequences"]):
+            got = oracle_lib.offsetgen_sequence(oracle, "orc", *args, state, 0, rand_algo=algo_id)
+            assert [list(x) for x in got] == seq, (algo_id, args[0])
 
 
 def test_offsetgen_golden(oracle, golden):
@@ -196,47 +196,28 @@ def test_offsetgen_fullcoverage_covers_every_block(oracle):
     assert sorted(off for off, _ in seq) == [(first + i) * block for i in range(nblocks)]
 
 
-def test_offsetgen_live_vs_reference_headers(oracle, ref):
-    rng = random.Random(99)
-    for _ in range(60):
-        kind = rng.randrange(6)
-        block = rng.choice([512, 4096, 65536, 1000])
-        nblocks = rng.randrange(1, 50)
-        length = nblocks * block + (rng.randrange(block) if kind in (0, 1, 2, 3) else 0)
-        offset = rng.randrange(0, 100) * block
-        total = rng.randrange(1, 80) * block + rng.choice([0, 0, 17])
-        if kind == oracle_lib.OFFGEN_FULLCOV:
-            # only the first permutation cycle is reproducible: the reference re-seeds every
-            # further cycle from std::random_device (FullCoverageV2.h:155-164)
-            length = nblocks * block
-            total = min(total - total % block, length) or block
-        threads = rng.randrange(1, 5)
-        state = [rng.getrandbits(64) for _ in range(4)]
-        lcg = rng.getrandbits(32)
-        a = oracle_lib.offsetgen_sequence(oracle, "orc", kind, total, length, offset, block,
-                                          threads, state, lcg)
-        b = oracle_lib.offsetgen_sequence(ref, "ref", kind, total, length, offset, block, threads,
-                                          state, lcg)
-        assert a == b, (kind, total, length, offset, block)
+def test_offsetgen_live_vs_reference_headers(oracle, recorded):
+    """random geometries, states and seeds of all six generators against the answers of the
+    reference's headers (recorded by tests/golden/make_golden.py)"""
+    cases = make_golden.offsetgen_cases()
+    assert len(cases) == len(recorded["offsetgen"])
+    for case, want in zip(cases, recorded["offsetgen"]):
+        got = oracle_lib.offsetgen_sequence(oracle, "orc", *case)
+        assert [list(x) for x in got] == want, case[:6]
 
 
-def test_prngs_live_vs_reference_headers(oracle, ref):
-    rng = random.Random(5)
-    for _ in range(10):
-        state = [rng.getrandbits(64) for _ in range(4)]
-        seed = rng.getrandbits(64)
-        length = rng.choice([0, 1, 8, 100, 262144, 262145, 700001])
-        algo = ref.ref_goldenprime_create(seed, oracle_lib.u64x4(state))
-        rbuf = ctypes.create_string_buffer(max(1, length))
-        ref.ref_randalgo_fill_buf(algo, rbuf, length)
-        rnext = ref.ref_randalgo_next(algo)
-        ref.ref_randalgo_destroy(algo)
+def test_prngs_live_vs_reference_headers(oracle, recorded):
+    """golden prime buffer fills against the answers of the reference's headers (recorded by
+    tests/golden/make_golden.py)"""
+    cases = make_golden.goldenprime_cases()
+    assert len(cases) == len(recorded["goldenprime"])
+    for (state, seed, length), want in zip(cases, recorded["goldenprime"]):
         st = oracle_lib.GoldenPrime()
         oracle.orc_goldenprime_init(ctypes.byref(st), seed, oracle_lib.u64x4(state))
         obuf = ctypes.create_string_buffer(max(1, length))
         oracle.orc_goldenprime_fill_buf(ctypes.byref(st), obuf, length)
-        assert obuf.raw[:length] == rbuf.raw[:length]
-        assert oracle.orc_goldenprime_next(ctypes.byref(st)) == rnext
+        assert hashlib.sha256(obuf.raw[:length]).hexdigest() == want["fill_sha256"], length
+        assert oracle.orc_goldenprime_next(ctypes.byref(st)) == want["next_after_fill"]
 
 
 def test_rand_refill_layout(oracle):

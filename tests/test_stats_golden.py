@@ -5,12 +5,11 @@ restatement and the product's C ABI must both reproduce them."""
 import ctypes
 import json
 import os
-import random
 
 import pytest
 
 from elbencho_b200._native import Histogram
-from tests import oracle_lib
+from tests.golden import make_golden
 
 GOLDEN_PATH = os.path.join(os.path.dirname(__file__), "golden", "ref_vectors.json")
 
@@ -86,43 +85,35 @@ def test_oracle_per_sec_matches_reference(oracle, golden):
         assert oracle.orc_per_sec_from_usec(total, usec) == want
 
 
-def test_live_against_reference_headers(native, oracle, ref):
-    """random latency sets, merged pairwise: product == oracle == the reference's class"""
-    rng = random.Random(11)
-    for _ in range(20):
-        parts = []
-        for _ in range(2):
-            lats = [int(rng.random() ** rng.choice([1, 4]) * rng.choice([50, 10 ** 4, 10 ** 7]))
-                    for _ in range(rng.randrange(0, 300))]
+def test_live_against_reference_headers(native, oracle, recorded):
+    """random latency sets, merged pairwise: product == oracle == the reference's class (its
+    answers recorded by tests/golden/make_golden.py)"""
+    cases = make_golden.histogram_merge_cases()
+    assert len(cases) == len(recorded["histogram_merges"])
+    for parts, want in zip(cases, recorded["histogram_merges"]):
+        histos = []
+        for lats in parts:
             mine, orc = Histogram(), Histogram()
             native.elb_histogram_reset(ctypes.byref(mine))
             oracle.orc_histogram_reset(ctypes.byref(orc))
-            theirs = ref.ref_histogram_create()
             for lat in lats:
                 native.elb_histogram_add_latency(ctypes.byref(mine), lat)
                 oracle.orc_histogram_add_latency(ctypes.byref(orc), lat)
-                ref.ref_histogram_add(theirs, lat)
-            parts.append((mine, orc, theirs))
-        native.elb_histogram_merge(ctypes.byref(parts[0][0]), ctypes.byref(parts[1][0]))
-        oracle.orc_histogram_merge(ctypes.byref(parts[0][1]), ctypes.byref(parts[1][1]))
-        ref.ref_histogram_merge(parts[0][2], parts[1][2])
-        mine, orc, theirs = parts[0]
-        buckets = (ctypes.c_uint64 * ref.ref_histogram_num_buckets(theirs))()
-        ref.ref_histogram_buckets(theirs, buckets)
-        assert list(mine.buckets) == list(orc.buckets) == list(buckets)
+            histos.append((mine, orc))
+        native.elb_histogram_merge(ctypes.byref(histos[0][0]), ctypes.byref(histos[1][0]))
+        oracle.orc_histogram_merge(ctypes.byref(histos[0][1]), ctypes.byref(histos[1][1]))
+        mine, orc = histos[0]
+        assert list(mine.buckets) == list(orc.buckets) == want["buckets"]
         for histo in (mine, orc):
-            assert histo.numStoredValues == ref.ref_histogram_num(theirs)
-            assert histo.numMicroSecTotal == ref.ref_histogram_sum(theirs)
+            assert histo.numStoredValues == want["num"]
+            assert histo.numMicroSecTotal == want["sum"]
             if histo.numStoredValues:
-                assert histo.minMicroSecLat == ref.ref_histogram_min(theirs)
-                assert histo.maxMicroSecLat == ref.ref_histogram_max(theirs)
+                assert histo.minMicroSecLat == want["min"]
+                assert histo.maxMicroSecLat == want["max"]
         if mine.numStoredValues:
-            for pct in (10.0, 50.0, 99.0):
-                want = ref.ref_histogram_percentile(theirs, pct)
-                assert native.elb_histogram_percentile(ctypes.byref(mine), pct) == \
-                    pytest.approx(want, rel=1e-12)
-        for _, _, handle in parts:
-            ref.ref_histogram_destroy(handle)
+            for pct, value in want["percentiles"].items():
+                assert native.elb_histogram_percentile(ctypes.byref(mine), float(pct)) == \
+                    pytest.approx(value, rel=1e-12)
 
 
 def test_service_password_hash_matches_reference(native, golden):
