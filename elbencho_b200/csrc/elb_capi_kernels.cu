@@ -30,6 +30,21 @@ static int checkRandArgs(unsigned pct, int randAlgo)
 	return 0;
 }
 
+/* the staged kernels move 32-byte vectors between (devPtr) and (devPtr + hostDelta): both ends of
+   a vector are aligned only if hostDelta is */
+static int checkHostDelta(const char* what, int64_t hostDelta)
+{
+	if(hostDelta % ELB_STAGE_ALIGN)
+	{
+		elb_set_last_error(std::string(what) + ": hostDelta must be a multiple of " +
+			std::to_string(ELB_STAGE_ALIGN) + " bytes (alignment of the staged vector copies). "
+			"Given: " + std::to_string(hostDelta) );
+		return -1;
+	}
+
+	return 0;
+}
+
 extern "C" {
 
 int elb_abi_version(void)
@@ -157,6 +172,9 @@ int elb_fill_pattern_staged(const elb_block_desc* descs, uint32_t numDescs, uint
 	int64_t hostDelta, uint64_t* devCounters, uint64_t totalBytes, uint64_t maxBlockLen,
 	void* stream)
 {
+	if(checkHostDelta("elb_fill_pattern_staged", hostDelta) )
+		return -1;
+
 	if(numDescs && !descs)
 	{
 		elb_set_last_error("elb_fill_pattern_staged: NULL descriptor array");
@@ -174,6 +192,9 @@ int elb_fill_random_staged(const elb_block_desc* descs, uint32_t numDescs, unsig
 	uint64_t seed, int randAlgo, int64_t hostDelta, uint64_t* devCounters, uint64_t totalBytes,
 	uint64_t maxBlockLen, void* stream)
 {
+	if(checkHostDelta("elb_fill_random_staged", hostDelta) )
+		return -1;
+
 	if(checkRandArgs(pct, randAlgo) )
 		return -1;
 
@@ -195,6 +216,9 @@ int elb_verify_pattern_staged(const elb_block_desc* descs, uint32_t numDescs, ui
 	unsigned* devDoneTicket, uint64_t* devCounters, uint64_t totalBytes, uint64_t maxBlockLen,
 	void* stream)
 {
+	if(checkHostDelta("elb_verify_pattern_staged", hostDelta) )
+		return -1;
+
 	if(numDescs && (!descs || !devResults) )
 	{
 		elb_set_last_error("elb_verify_pattern_staged: NULL descriptor or result array");
@@ -213,6 +237,9 @@ int elb_verify_pattern_staged(const elb_block_desc* descs, uint32_t numDescs, ui
 int elb_stage_copy(const elb_block_desc* descs, uint32_t numDescs, int hostToDevice,
 	int64_t hostDelta, uint64_t totalBytes, uint64_t maxBlockLen, void* stream)
 {
+	if(checkHostDelta("elb_stage_copy", hostDelta) )
+		return -1;
+
 	if(!numDescs)
 		return 0;
 

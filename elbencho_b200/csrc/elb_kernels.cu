@@ -318,9 +318,11 @@ __device__ __forceinline__ void copy_tile(const BlockGeom& g, uint64_t tileIdx, 
 
 /* ---- verify ----------------------------------------------------------------------------- */
 
-/* compare one 32-byte vector; update thread-local count and first mismatch position */
+/* compare one 32-byte vector; update thread-local count and first mismatch position (Count: 32
+ * bits where the count covers one tile, 64 bits where it covers a whole block of any length) */
+template<class Count>
 __device__ __forceinline__ void verify_vec(const u64x4& got, const u64x4& exp, uint64_t pos,
-	unsigned& numBad, uint64_t& firstBad)
+	Count& numBad, uint64_t& firstBad)
 {
 	const uint64_t anyDiff = (got.a ^ exp.a) | (got.b ^ exp.b) | (got.c ^ exp.c) |
 		(got.d ^ exp.d);
@@ -834,7 +836,9 @@ __device__ __forceinline__ void process_block_warp(const KernelArgs& args, const
 	uint8_t* devBody = g.ptr + g.headLen;
 	uint8_t* hostBody = devBody + hostDelta;
 
-	unsigned numBad = 0;
+	/* 64 bits: the warp walks the whole block, and a block may be longer than the size hint that
+	   picked this kernel, so the count of one warp is not bounded by 32 bits */
+	unsigned long long numBad = 0;
 	uint64_t firstBad = ~0ULL;
 
 	for(uint64_t spanStart = 0; spanStart < g.bodyLen; spanStart += ELB_WARP_SPAN)
@@ -934,10 +938,14 @@ __device__ __forceinline__ void process_block_warp(const KernelArgs& args, const
 
 	if(MODE == MODE_VERIFY_PATTERN)
 	{
-		const unsigned warpBad = __reduce_add_sync(0xffffffffu, numBad);
+		const unsigned anyBad = __reduce_or_sync(0xffffffffu, numBad ? 1u : 0u);
 
-		if(__builtin_expect(warpBad != 0, 0) )
+		if(__builtin_expect(anyBad != 0, 0) )
 		{
+			unsigned long long warpBad = numBad; // (redux adds 32 bits only)
+			for(int laneMask = 16; laneMask; laneMask >>= 1)
+				warpBad += __shfl_xor_sync(0xffffffffu, warpBad, laneMask);
+
 			const unsigned firstHi = (unsigned)(firstBad >> 32);
 			const unsigned minHi = __reduce_min_sync(0xffffffffu, firstHi);
 			const unsigned firstLo = (firstHi == minHi) ? (unsigned)firstBad : 0xffffffffu;

@@ -179,7 +179,12 @@ int elb_fill_random_batch_sized(const elb_block_desc* descs, uint32_t numDescs, 
  *                     are given, the last CTA of the launch copies the per-block results to
  *                     hostResults (pinned) and re-arms the device entries.
  *   stage_copy      : plain copy host -> device (hostToDevice != 0) or device -> host
- * hostDelta == 0 turns the staging off (verify then still publishes to hostResults). */
+ * hostDelta == 0 turns the staging off (verify then still publishes to hostResults).
+ * hostDelta must be a multiple of ELB_STAGE_ALIGN (32): the kernels move 32-byte vectors, and both
+ * ends of a vector are aligned only then. Page-aligned rings of equal layout satisfy this. Any
+ * other hostDelta is rejected with -1 before anything is launched. */
+#define ELB_STAGE_ALIGN 32
+
 int elb_fill_pattern_staged(const elb_block_desc* descs, uint32_t numDescs, uint64_t salt,
 	int64_t hostDelta, uint64_t* devCounters, uint64_t totalBytes, uint64_t maxBlockLen,
 	void* stream);

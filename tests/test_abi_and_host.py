@@ -261,3 +261,25 @@ def test_nodiocheck_skips_the_direct_io_block_size_check(native):
     finally:
         if os.path.exists(common["paths"][0]):
             os.unlink(common["paths"][0])
+
+
+@pytest.mark.parametrize("host_delta", [4, -8])
+def test_staged_entry_points_reject_misaligned_host_delta(native, host_delta):
+    """the staged kernels move 32-byte vectors to / from (devPtr + hostDelta): a hostDelta that is
+    not a multiple of 32 is refused by the argument check, before anything reaches the GPU"""
+    desc = _native.BlockDesc()  # never read: the check comes first
+    ptr = ctypes.cast(ctypes.pointer(desc), ctypes.c_void_p)
+    calls = {
+        "elb_fill_pattern_staged": lambda: native.elb_fill_pattern_staged(
+            ptr, 1, 1, host_delta, None, 4096, 4096, None),
+        "elb_fill_random_staged": lambda: native.elb_fill_random_staged(
+            ptr, 1, 50, 1, 0, host_delta, None, 4096, 4096, None),
+        "elb_verify_pattern_staged": lambda: native.elb_verify_pattern_staged(
+            ptr, 1, 1, host_delta, ptr, None, None, None, 4096, 4096, None),
+        "elb_stage_copy": lambda: native.elb_stage_copy(ptr, 1, 1, host_delta, 4096, 4096, None),
+    }
+    for name, call in calls.items():
+        assert call() == -1, name
+        err = _native.last_error()
+        assert err.startswith(name + ": hostDelta must be a multiple of 32"), err
+        assert "Given: %d" % host_delta in err

@@ -593,3 +593,44 @@ def test_small_block_staged_kernels(cuda_device):
     for ptr, n, _, _ in blocks:
         lo = ptr - dev.data_ptr()
         assert host_b[lo:lo + n] == dev_b[lo:lo + n]
+
+
+# ------------------------------------------------------------------------------------------------
+# 64-bit edges: one block longer than 2^32 bytes
+# ------------------------------------------------------------------------------------------------
+
+@pytest.mark.parametrize("shape", ["warp", "tiled", "persistent"])
+def test_block_longer_than_4gib_counts_and_locates_in_64_bits(cuda_device, shape):
+    """a single block of 4 GiB + 16 KiB + 5 through each launch shape (picked by the size hints;
+    the warp kernel walks a block longer than its hint completely): a count of every byte must not
+    wrap at 2^32, and a first mismatch beyond 2^32 takes the high word of the 64-bit minimum"""
+    length = 2 ** 32 + 16 * 1024 + 5
+    salt = 0x1122334455667788
+    other_salt = (salt + 0x0101010101010101) % 2 ** 64  # differs from salt in every byte
+    hints = {"warp": dict(total_bytes=length, max_block_len=4096),
+             "tiled": dict(total_bytes=length, max_block_len=length),
+             "persistent": {}}[shape]
+    buf = torch.empty(length, dtype=torch.uint8, device=cuda_device)
+    try:
+        descs = make_batch(cuda_device, [(buf.data_ptr(), length, 0, 0)])
+        results = torch.zeros(2, dtype=torch.int64, device=cuda_device)
+        counters = torch.zeros(kernels.DEVCTR_NUM, dtype=torch.int64, device=cuda_device)
+        kernels.fill_pattern_batch(descs.data_ptr(), 1, salt, 0, stream_handle(),
+                                   total_bytes=length, max_block_len=length)
+        kernels.verify_pattern_batch(descs.data_ptr(), 1, other_salt, results.data_ptr(),
+                                     counters.data_ptr(), stream_handle(), **hints)
+        torch.cuda.synchronize()
+        assert read_result(results) == [(length, 0)]
+        ctr = counters.cpu().tolist()
+        assert ctr[kernels.DEVCTR_VERIFY_MISMATCH_BYTES] == length
+        assert ctr[kernels.DEVCTR_VERIFIED_BYTES] == length
+
+        bad = 2 ** 32 + 12345
+        buf[bad] ^= 0x10
+        kernels.verify_pattern_batch(descs.data_ptr(), 1, salt, results.data_ptr(), 0,
+                                     stream_handle(), **hints)
+        torch.cuda.synchronize()
+        assert read_result(results) == [(1, bad)]
+    finally:
+        del buf
+        torch.cuda.empty_cache()
